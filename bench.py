@@ -14,6 +14,8 @@ Contract: `python bench.py --gpus N --steps K --warmup W [--impl reference]`, on
   cpu_baseline = the CPU oracle (reference runtime objects + restated pipelines, NOT the LLVM JIT) on the box's host cores
             over a bounded sample of the same table.
 `--impl reference` times that CPU implementation alone on the same config (rank 0 only).
+`--dump-outputs DIR` writes the Q1 rows of the last timed step as DIR/<column>.npy (float64): the inputs are generated from
+`--seed`, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -51,6 +53,7 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the full-size oracle gates (profiling runs only)")
     ap.add_argument("--no-extra", action="store_true", help="skip the Q6/Q3/Q5/Q9 entries")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the Q1 result rows of the last timed step as DIR/<column>.npy (float64)")
     return ap.parse_args()
 
 
@@ -251,6 +254,20 @@ def q1_sums(rows):
     return {(r["l_returnflag"], r["l_linestatus"]): (r["sum_qty"], r["sum_base_price"], r["sum_disc_price"], r["sum_charge"], r["count_order"]) for r in rows}
 
 
+# decimal scale of each Q1 result column (sums of products add the factors' scales, averages are decimal(31,21))
+Q1_RESULT_SCALES = {"l_returnflag": 0, "l_linestatus": 0, "sum_qty": 2, "sum_base_price": 2, "sum_disc_price": 4, "sum_charge": 6,
+                    "avg_qty": 21, "avg_price": 21, "avg_disc": 21, "count_order": 0}
+
+
+def dump_q1_rows(out_dir, rows):
+    """One float64 array per Q1 result column, in result order: decimals as the numbers they stand for, the two flags as their
+    fixed_size_binary(4) cells read as int32.  Two builds of the project compare output for output on the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, scale in Q1_RESULT_SCALES.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.array([r[name] / 10**scale for r in rows], dtype=np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -383,6 +400,8 @@ def run_ours(args):
     torch.cuda.synchronize()
     wall_ms = 1000 * (time.perf_counter() - t0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # every rank holds the same merged rows
+        dump_q1_rows(args.dump_outputs, rows)
     barrier()
     launches = ctx.launch_count() - launches0
     k_ms, k_n = ctx.kernel_time("scan_groupby")

@@ -80,19 +80,28 @@ class _Lock:
 
 
 def build_datagen_host(verbose=False, force=False):
+    # an up-to-date library is returned without the lock: loading must work from a read-only tree
+    if not force and _up_to_date(GEN_LIB, _datagen_host_stamp()):
+        return GEN_LIB
     with _Lock():
         return _build_datagen_host(verbose, force)
 
 
 def build_gpu(verbose=False, force=False, ptxas_verbose=False):
+    if not force and _up_to_date(GPU_LIB, _gpu_stamp()):
+        return GPU_LIB
     with _Lock():
         return _build_gpu(verbose, force, ptxas_verbose)
 
 
+def _datagen_host_stamp():
+    deps = [os.path.join(CSRC, f) for f in ("datagen_host.cpp", "tpch_gen.h", "dbgen_gen.h")] + [os.path.join(INCLUDE, "ldb_datagen.h")]
+    return _stamp(deps)
+
+
 def _build_datagen_host(verbose=False, force=False):
     srcs = [os.path.join(CSRC, "datagen_host.cpp")]
-    deps = srcs + [os.path.join(CSRC, "tpch_gen.h"), os.path.join(CSRC, "dbgen_gen.h"), os.path.join(INCLUDE, "ldb_datagen.h")]
-    stamp = _stamp(deps)
+    stamp = _datagen_host_stamp()
     if not force and _up_to_date(GEN_LIB, stamp):
         return GEN_LIB
     _run([CXX, "-std=c++17", "-O3", "-fPIC", "-pthread", "-shared", "-Wall", "-I", INCLUDE, "-o", GEN_LIB] + srcs, verbose)
@@ -100,12 +109,22 @@ def _build_datagen_host(verbose=False, force=False):
     return GEN_LIB
 
 
-def _build_gpu(verbose=False, force=False, ptxas_verbose=False):
+def _gpu_sources():
     cu = _sources((".cu",))
     cpp = [p for p in _sources((".cpp",)) if not p.endswith("_host.cpp")]
     host_cpp = [p for p in _sources((".cpp",)) if p.endswith("_host.cpp") and not p.endswith("datagen_host.cpp")]  # g++ only (function multi-versioning)
     hdr = _sources((".h", ".cuh")) + [os.path.join(INCLUDE, f) for f in sorted(os.listdir(INCLUDE))]
-    stamp = _stamp(cu + cpp + host_cpp + hdr, " ".join(NVCC_FLAGS).replace(ROOT, "$ROOT"))
+    return cu, cpp, host_cpp, hdr
+
+
+def _gpu_stamp():
+    cu, cpp, host_cpp, hdr = _gpu_sources()
+    return _stamp(cu + cpp + host_cpp + hdr, " ".join(NVCC_FLAGS).replace(ROOT, "$ROOT"))
+
+
+def _build_gpu(verbose=False, force=False, ptxas_verbose=False):
+    cu, cpp, host_cpp, _ = _gpu_sources()
+    stamp = _gpu_stamp()
     if not force and _up_to_date(GPU_LIB, stamp):
         return GPU_LIB
     objdir = os.path.join(HERE, "build")
@@ -144,11 +163,13 @@ def _build_gpu(verbose=False, force=False, ptxas_verbose=False):
 
 def build_arrow_io(verbose=False, force=False):
     """libldb_arrow_io.so: Arrow IPC file → backend table (csrc_arrow/), linked against the Arrow C++ that ships inside pyarrow."""
+    import pyarrow
+    src = os.path.join(HERE, "csrc_arrow", "arrow_table_io.cpp")
+    deps = [src, os.path.join(INCLUDE, "ldb_arrow_io.h"), os.path.join(INCLUDE, "ldb_gpu.h")]
+    if not force and _up_to_date(ARROW_LIB, _stamp(deps, pyarrow.__version__)):
+        return ARROW_LIB
     with _Lock():
-        import pyarrow
         pa_dir = os.path.dirname(pyarrow.__file__)
-        src = os.path.join(HERE, "csrc_arrow", "arrow_table_io.cpp")
-        deps = [src, os.path.join(INCLUDE, "ldb_arrow_io.h"), os.path.join(INCLUDE, "ldb_gpu.h")]
         stamp = _stamp(deps, pyarrow.__version__)
         if not force and _up_to_date(ARROW_LIB, stamp):
             return ARROW_LIB

@@ -10,6 +10,8 @@ import pytest
 from lingodb_b200 import datagen
 from oracle import oracle as O
 
+import _reference_answers as R
+
 GOLD = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "reference_kats.json")))
 M64 = 2**64
 
@@ -120,7 +122,7 @@ def _cols(t, names):
 
 @pytest.fixture(scope="module")
 def tables():
-    return datagen.tpch(0.03, seed=9, chunk_rows=5000)
+    return R.tpch_tables()
 
 
 def test_q6_and_q1_match_numpy(orc, tables):
@@ -185,22 +187,14 @@ def test_q3_and_q5_match_python(orc, tables):
 
 
 def test_port_equals_reference_objects(tables):
-    if not os.path.exists(O.REF_LIB):
-        pytest.skip("oracle/_ref not built (no /root/reference): parity of the port is pinned by the KATs only")
-    res = []
-    for kind in ("port", "reference"):
-        o = O.Oracle(kind, workers=4)
-        h = {k: o.table(v) for k, v in tables.items()}
-        res.append((o.q6(h["lineitem"])[0], o.q1(h["lineitem"])[0], o.q3(h["customer"], h["orders"], h["lineitem"])[0],
-                    o.q5(h["customer"], h["orders"], h["lineitem"], h["supplier"], h["nation"], h["region"])[0]))
-    assert res[0] == res[1]
-    t9 = datagen.tpch(0.02, seed=4, chunk_rows=3000, with_parts=True)
-    res9 = []
-    for kind in ("port", "reference"):
-        o = O.Oracle(kind, workers=4)
-        h = {k: o.table(v) for k, v in t9.items()}
-        res9.append(o.q9(h["part"], h["supplier"], h["lineitem"], h["partsupp"], h["orders"], h["nation"])[0])
-    assert res9[0] == res9[1] and len(res9[0]) > 150
+    """The port answers as the reference's own runtime objects do: against their stored answers always, and against the
+    reference-compiled build itself where oracle/_ref is built."""
+    want = R.stored()["tpch"]
+    assert len(want["q9"]) > 150
+    for kind in (["port", "reference"] if os.path.exists(O.REF_LIB) else ["port"]):
+        got = R.tpch_answers(O.Oracle(kind, workers=4), tables)
+        for q in ("q6", "q1", "q3", "q5", "q9"):
+            assert got[q] == want[q], (kind, q)
 
 
 def test_oracle_edge_cases(orc):
